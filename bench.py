@@ -93,6 +93,9 @@ def parse_args():
                     help="N > 1: resident fusion CTAs per SM (KB_FUSE_CTAS_PER_SM; 0 = library default = full occupancy). Fewer CTAs leave "
                          "registers for the next batch's block selection / culling kernels to run beside the fusion kernel")
     ap.add_argument("--small", action="store_true", help="tiny configuration for functional checks")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="1 GPU, hall workloads: after the timed steps, write the map they produced as DIR/<name>.npy (every "
+                         "block index, and the voxels of a fixed seeded sample of the blocks), so that two builds can be compared")
     ap.add_argument("--workload", default="hall640", choices=["hall640", "hall1280", "dynamic"],
                     help="hall640 = BASELINE config[1] (fusion only, the headline, used for every --gpus N); hall1280 = "
                          "config[3] shapes (1280x720, 2 cm voxels: ~20x the voxel work per frame) for the sharded "
@@ -562,6 +565,45 @@ def combine_checksums(parts):
             "blocks": int(sum(int(p[2]) for p in parts)), "observed_voxels": int(sum(int(p[3]) for p in parts))}
 
 
+DUMP_SAMPLE_BLOCKS = 512  # voxels of 512 blocks: 40 MB, inside the 64 MB the dump may take
+DUMP_SEED = 0
+
+
+def dump_outputs(h, out_dir):
+    """Writes the map as a caller reads it back (kb_export_blocks, blocks ascending in (x, y, z)): the index of every block,
+    and the TSDF, semantic label (-1 where the voxel has none) and last_observed stamp of every voxel of a fixed seeded
+    sample of the blocks. The sample is drawn by position in the sorted block list, so two builds that compute the same
+    map dump the same blocks. One field is exported per call to bound host memory (the whole map is GBs)."""
+    from khronos_b200 import capi
+    n, V = h.num_blocks(), h.V
+
+    def field(name, dtype, width):
+        a = np.zeros((n, width), dtype)
+        ex = capi.BlockExport()
+        setattr(ex, name, a.ctypes.data)
+        nw = ctypes.c_int32(0)
+        if n:
+            h._check(h._fn("export_blocks")(h._h, capi.EXPORT_ALL, n, ctypes.byref(ex), ctypes.byref(nw)))
+            assert nw.value == n
+        return a
+
+    index = field("block_index", np.int32, 3)
+    sel = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(DUMP_SAMPLE_BLOCKS, n), replace=False))
+    empty = field("semantic_empty", np.uint8, V)[sel]
+    out = {
+        "block_index": index.astype(np.float64),
+        "sample_block_index": index[sel].astype(np.float64),
+        "sample_distance": field("distance", np.float32, V)[sel],
+        "sample_weight": field("weight", np.float32, V)[sel],
+        "sample_semantic_label": np.where(empty != 0, -1.0, field("semantic_label", np.uint32, V)[sel]).astype(np.float32),
+        "sample_last_observed_ns": field("last_observed", np.uint64, V)[sel].astype(np.float64),  # exact below 2^53 ns
+    }
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main_hall_cells(args, world, rank, local_rank, dev):
     """N > 1, --shard cells (khronos_b200/replay.py): cell-sharded map, stream striped over the ranks' frame pools, every
     rank pulls the frames whose frustum touches its cells over NVLink (CUDA IPC peer mappings) and fuses its sub-sequence
@@ -870,6 +912,8 @@ def main_hall_cells(args, world, rank, local_rank, dev):
 def main():
     args = parse_args()
     quiet_stdout()
+    if args.dump_outputs and (args.impl != "b200" or args.workload == "dynamic" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        raise SystemExit("bench.py: --dump-outputs covers the single-GPU hall workloads (--impl b200, 1 GPU, not --workload dynamic)")
     if args.impl == "reference":
         return main_reference(args)
     if args.workload == "dynamic":
@@ -1101,6 +1145,8 @@ def main():
         raise SystemExit("bench.py: block pool exhausted (capacity_exceeded): results incomplete")
     # order-independent checksum of the map after the timed region (same value for every --gpus N: the bench verifies itself)
     cs = h.map_checksum()
+    if args.dump_outputs:  # before the e2e windows and legs below, which integrate more frames into this map
+        dump_outputs(h, args.dump_outputs)
     pairs = t64_1.block_frame_pairs - t64_0.block_frame_pairs
     n_frames = K * F
     # 64-bit cumulative counters (kb_get_totals64): the 32-bit ones wrap after ~36 k frames of this workload

@@ -1,4 +1,5 @@
-"""bench.py's pure helpers (no GPU): byte model, checksum combination, group counting, roofline block arithmetic."""
+"""bench.py's helpers (no GPU): byte model, checksum combination, group counting, roofline block arithmetic, the map
+sample written by --dump-outputs."""
 import argparse
 import importlib.util
 import os
@@ -41,3 +42,35 @@ def test_roofline_block_fraction():
     assert abs(r["frac"] - r["achieved"] / r["peak"]) < 1e-12 and 0.1 < r["frac"] < 0.5
     assert abs(r["launch_us"] - 28000.0 / 157) < 1e-9 and r["unit"] == "GB/s" and r["bound"] == "hbm"
     assert abs(r["algorithmic_bytes_per_launch"] - total / 157) < 1.0
+
+
+def test_dump_outputs_is_a_sample_of_the_exported_map(oracle_lib, tmp_path, monkeypatch):
+    """--dump-outputs on a map behind the same C ABI (the oracle's): every block index, and the voxels of the sampled
+    blocks exactly as kb_export_blocks returns them; float32 / float64 only; the same sample on every run."""
+    import numpy as np
+    import harness as hs
+    from khronos_b200 import synthetic as syn
+    b = _bench()
+    cam = hs.small_camera(4)
+    poses, stamps = syn.orbit_trajectory(4, laps=0.05)
+    h = hs.make_handle(oracle_lib, "ko_", cam=cam)
+    hs.run_fusion(h, hs.render_frames(syn.room_scene(), cam, poses, stamps), poses, stamps, tracking=True)
+    ex = h.export_blocks(likelihoods=False)
+    monkeypatch.setattr(b, "DUMP_SAMPLE_BLOCKS", ex.n // 3)
+    b.dump_outputs(h, str(tmp_path / "a"))
+    b.dump_outputs(h, str(tmp_path / "b"))
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) and len(names) == 6
+    d = {n[:-4]: np.load(tmp_path / "a" / n) for n in names}
+    for n in names:
+        np.testing.assert_array_equal(d[n[:-4]], np.load(tmp_path / "b" / n))
+        assert d[n[:-4]].dtype in (np.float32, np.float64)
+    np.testing.assert_array_equal(d["block_index"], ex.block_index)
+    pos = [int(np.flatnonzero((ex.block_index == r).all(1))[0]) for r in d["sample_block_index"]]
+    assert len(pos) == ex.n // 3 and pos == sorted(set(pos))
+    np.testing.assert_array_equal(d["sample_distance"], ex.distance[pos])
+    np.testing.assert_array_equal(d["sample_weight"], ex.weight[pos])
+    np.testing.assert_array_equal(d["sample_last_observed_ns"], ex.last_observed[pos].astype(np.float64))
+    lab = np.where(ex.semantic_empty[pos] != 0, -1, ex.semantic_label[pos].astype(np.int64))
+    np.testing.assert_array_equal(d["sample_semantic_label"], lab)
+    assert (d["sample_weight"] > 0).any() and (d["sample_semantic_label"] >= 0).any()
